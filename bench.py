@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ANI-2x energy+force hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--config NAME]     # B200 arm (this repo)
+    python bench.py --gpus N --steps K --warmup W [--config NAME] [--dump-outputs DIR]     # B200 arm (this repo)
     python bench.py --impl reference --steps K --warmup W [--config NAME]
                                       # reference arm: the UNMODIFIED aiqm/torchani on the host cores
 
@@ -42,6 +42,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -233,7 +234,14 @@ def main():
     ap.add_argument("--skin", type=float, default=0.0,
                     help="experiment: Verlet skin (A) of the end-to-end arm; the atoms then move ballistically "
                          "(300 K Maxwell-Boltzmann velocities, 1 fs per step) so that grid reuse is exercised")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each timed path returned as DIR/<name>.npy (rank 0): "
+                         "energies (f64) and grad = dE/dcoords (f32) of the device step, e2e_energies (f64) and "
+                         "e2e_forces (f32) of the host-buffer step; the inputs are seeded, so two builds can be "
+                         "compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -306,10 +314,12 @@ def main():
         flush.fill_(1)
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        one_step()
+        out = one_step()
         b.record()
         evs.append((a, b))
     barrier()
+    # copied now: the step's result tensors are workspace buffers that later steps overwrite
+    dumps = {"energies": out[0].cpu().numpy(), "grad": out[1].cpu().numpy()}
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     t_all = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -327,7 +337,6 @@ def main():
                               skin=args.skin, sharded=sharded if world > 1 else None)
         h_pos = coords[0].numpy().copy()
         if args.skin > 0:   # A/fs: sqrt(kT/m), kT = 0.02585 eV, 1 amu A^2/fs^2 = 103.6427 eV
-            import numpy as np
             mass = np.where(z[0].numpy() == 1, 1.008, 15.999)[:, None]
             h_vel = (np.random.default_rng(0).normal(size=h_pos.shape) * np.sqrt(0.02585 / (103.6427 * mass))).astype("float32")
 
@@ -372,10 +381,12 @@ def main():
         flush.fill_(1)
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        e2e_step()
+        e2e_out = e2e_step()
         b.record()
         e2e_evs.append((a, b))
     barrier()
+    dumps["e2e_energies"] = np.array(e2e_out[0], dtype=np.float64).reshape(-1)
+    dumps["e2e_forces"] = np.array(e2e_out[1], dtype=np.float32)
     clocks = sampler.stop()
     e2e_ms = sum(a.elapsed_time(b) for a, b in e2e_evs)
     t_e2e = torch.tensor([e2e_ms], dtype=torch.float64, device=dev)
@@ -463,6 +474,10 @@ def main():
                 "operand_format": {"parts": fmt.parts, "bytes_per_element": 2 * fmt.parts},
                 "library_sha256_16": library_hash(), "library_build_id": library_build_id(),
                 "stage_ms": stage, "roofline": roofline, "roofline_aev": roofline_aev, "cpu_baseline": cpu}
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

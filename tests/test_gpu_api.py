@@ -562,3 +562,31 @@ def test_periodic_cell_thinner_than_the_cutoff_all_pairs_semantics():
     strict = models.from_weight_lists("2x", w32, device=DEV, neighborlist="cell_list", periodic_table_index=False)
     with pytest.raises(RuntimeError, match="too small"):
         strict((species.to(DEV), coords.float().to(DEV)), cell.float().to(DEV), pbc.to(DEV))
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: the last timed step of both timed paths, written as .npy, is the energy and force
+    of the seeded workload (checked against the float64 oracle), and --steps is the number of timed steps."""
+    import json
+    import subprocess
+    import sys
+    from helpers import ROOT
+    out = tmp_path / "dump"
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "water1k", "--molecules", "100",
+                          "--steps", "2", "--warmup", "3", "--cpu-steps", "0", "--dump-outputs", str(out)],
+                         capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
+    assert res.returncode == 0, res.stderr[-3000:]
+    line = json.loads(res.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["config"]["atoms"] == 300
+    d = {p.stem: np.load(p) for p in out.glob("*.npy")}
+    assert sorted(d) == ["e2e_energies", "e2e_forces", "energies", "grad"]
+    assert d["energies"].dtype == np.float64 and d["energies"].shape == (1,)
+    assert d["grad"].dtype == np.float32 and d["grad"].shape == (1, 300, 3)
+    assert d["e2e_energies"].dtype == np.float64 and d["e2e_forces"].dtype == np.float32
+    from torchani_b200 import synthetic
+    _, idx, coords, cell, pbc = synthetic.water_box(100, seed=0)
+    ref = orc.compute(oracle_model("2x", torch.float64), idx, coords.double(), cell.double(), pbc)
+    assert abs(float(d["energies"][0]) - float(ref["energy"][0])) < 5e-3             # float32 total
+    assert_close("forces", -d["grad"], ref["forces"].numpy(), 0.0, F_ATOL)
+    assert abs(float(d["e2e_energies"][0]) - float(ref["energy"][0])) < 5e-3
+    assert_close("e2e forces", d["e2e_forces"], ref["forces"][0].numpy(), 0.0, F_ATOL)

@@ -1,19 +1,19 @@
-"""Our AEV kernels against the REFERENCE'S OWN CUDA kernels (cuAEV), on the same GPU.
+"""Our AEV kernels against the REFERENCE'S OWN CUDA kernels (cuAEV).
 
-oracle/build_ref.sh compiles /root/reference/torchani/csrc/{aev.cu,cuaev.cpp} for sm_100 into
-oracle/_ref/cuaev.so (test infrastructure: git-ignored binary, travels to the GPU box; the reference's Python
-package does not travel, so the custom class / op are driven directly, exactly as aev/_computer.py:365-407 does).
-Checks the AEVs and the force-side gradient of the half-neighbour-list path (csrc/cuaev.cpp:204-223) and records
-how long the reference's kernels take beside ours (gpurun_out/ref_cuaev_timing.json when the directory exists).
-Skipped when the binary is absent (no /root/reference at build time) or does not load.
+The AEVs and the force-side gradient of the reference's half-neighbour-list path (csrc/cuaev.cpp:204-223) on seeded
+water boxes are stored in tests/golden/ref_cuaev_water*.npz (oracle/make_cuaev_golden.py, run on a B200 with the
+reference's kernels compiled for sm_100 by oracle/build_ref.sh); the first test checks ours against them.  The
+second test runs the reference's compiled cell list and cuAEV binaries (oracle/_ref, git-ignored) beside ours and
+records their times; it is skipped where those binaries are absent.
 """
 import json
 import os
 
+import numpy as np
 import pytest
 import torch
 
-from helpers import ROOT
+from helpers import GOLD, ROOT
 
 pytestmark = pytest.mark.gpu
 # one copy per process: the staged reference package (oracle/_ref/torchani, used by the drop-in tests) loads its own
@@ -52,65 +52,32 @@ def _time_ms(fn, reps=20, warm=5):
 
 @pytest.mark.parametrize("molecules", [333, 3333])
 def test_aev_and_gradient_match_the_reference_cuda_kernels(molecules):
-    from torchani_b200 import neighbors, synthetic
+    from torchani_b200 import synthetic
     from torchani_b200.aev import AEVComputer
-    from torchani_b200.engine import constants_2x
     dev = torch.device("cuda", 0)
-    consts = constants_2x()
-    comp = _reference_computer(consts, dev)
+    gold = np.load(os.path.join(GOLD, f"ref_cuaev_water{3 * molecules}.npz"))
+    rows = torch.from_numpy(gold["rows"]).to(dev)
+    aev_ref = torch.from_numpy(gold["aev"]).to(dev)
+    g_ref = torch.from_numpy(gold["grad"]).to(dev)
     _, idx, coords, cell, pbc = synthetic.water_box(molecules, seed=0)
     idx_d, cell_d, pbc_d = idx.to(dev), cell.to(dev), pbc.to(dev)
-    c_ref = coords.to(dev).requires_grad_(True)
-    nb = neighbors.CellList()(consts.rcr, idx_d, c_ref.detach(), cell_d, pbc_d)
-    ij32, diff, dist = nb.indices.to(torch.int32), nb.diff_vectors.contiguous(), nb.distances.contiguous()
-    sp32 = idx_d.to(torch.int32)
-
-    def ref_forward():
-        return torch.ops.cuaev.run_with_half_nbrlist(c_ref, sp32, ij32, diff, dist, comp)
-
-    aev_ref = ref_forward()
     ours = AEVComputer.like_2x().to(dev)
     c_our = coords.to(dev).requires_grad_(True)
     aev_our = ours(idx_d, c_our, cell_d, pbc_d)
-    assert aev_our.shape == aev_ref.shape
-    err = (aev_our - aev_ref).abs()
+    assert tuple(aev_our.shape) == tuple(gold["shape"])
+    err = (aev_our[0, rows] - aev_ref).abs()
     # two float32 GPU implementations of the same formulas (the reference with -use_fast_math)
     assert bool((err <= 5e-5 * aev_ref.abs() + 5e-5).all()), float(err.max())
-    g = torch.randn(aev_ref.shape, generator=torch.Generator().manual_seed(5)).to(dev)
-    (g_ref,) = torch.autograd.grad(aev_ref, c_ref, g)
+    g = torch.randn(aev_our.shape, generator=torch.Generator().manual_seed(5)).to(dev)
     (g_our,) = torch.autograd.grad(aev_our, c_our, g)
     scale = float(g_ref.abs().max())
     assert float((g_our - g_ref).abs().max()) <= 5e-4 * scale, (float((g_our - g_ref).abs().max()), scale)
 
-    if molecules == 3333:
-        # the reference's kernels beside ours (given pair list -> AEV -> gradient; ours includes the search)
-        def ref_fwd_bwd():
-            a = torch.ops.cuaev.run_with_half_nbrlist(c_ref, sp32, ij32, diff, dist, comp)
-            torch.autograd.grad(a, c_ref, g)
-
-        def our_fwd_bwd():
-            a = ours(idx_d, c_our, cell_d, pbc_d)
-            torch.autograd.grad(a, c_our, g)
-
-        with torch.no_grad():
-            t_ref_f = _time_ms(ref_forward)
-            t_our_f = _time_ms(lambda: ours(idx_d, c_our, cell_d, pbc_d))
-        rec = {"atoms": 3 * molecules, "pairs": int(ij32.shape[1]),
-               "reference_cuaev_forward_ms": t_ref_f, "reference_cuaev_forward_backward_ms": _time_ms(ref_fwd_bwd),
-               "ours_module_forward_ms": t_our_f, "ours_module_forward_backward_ms": _time_ms(our_fwd_bwd),
-               "note": "module-level API on both sides (torch tensors in and out, dense 1008-wide AEV written); the "
-                       "reference gets the pair list for free, ours builds its bucket grid inside the call"}
-        print("reference cuAEV vs ours:", json.dumps(rec))
-        out_dir = os.path.join(ROOT, "gpurun_out")
-        if os.path.isdir(out_dir):
-            with open(os.path.join(out_dir, "ref_cuaev_timing.json"), "w") as fh:
-                json.dump(rec, fh)
-
 
 def test_reference_gpu_path_pieces_beside_ours():
-    """The other two stages of the reference's GPU path on the same box and inputs: its C++/ATen cell list
-    (csrc/cell_list.cpp, built into oracle/_ref) and the BmmEnsemble network path (restated with torch.baddbmm in
-    oracle/gpu_baseline.py).  Checks that they agree with ours and records their times."""
+    """The stages of the reference's GPU path on the same box and inputs: its C++/ATen cell list
+    (csrc/cell_list.cpp, built into oracle/_ref), its cuAEV kernels and the BmmEnsemble network path (restated with
+    torch.baddbmm in oracle/gpu_baseline.py).  Checks that they agree with ours and records their times."""
     if os.environ.get("ANI_B200_REF_PATH_TEST", "0") == "0":
         pytest.skip("measurement of the reference's GPU path pieces: set ANI_B200_REF_PATH_TEST=1 to run it")
     from torchani_b200 import models, neighbors, synthetic
@@ -149,6 +116,29 @@ def test_reference_gpu_path_pieces_beside_ours():
     t_list_ref = _time_ms(ref_list, reps=5, warm=2)
     t_list_ours = _time_ms(lambda: neighbors.CellList()(consts.rcr, idx_d, c_d, cell_d, pbc_d), reps=5, warm=2)
 
+    # ---- AEV stage: the reference's cuAEV kernels (given pair list -> AEV -> gradient) vs our AEV module (which
+    #      builds its bucket grid inside the call); module-level API on both sides, dense 1008-wide AEV written
+    from torchani_b200.aev import AEVComputer
+    c_ref, c_our = c_d.clone().requires_grad_(True), c_d.clone().requires_grad_(True)
+    ij32, sp32 = ours_nb.indices.to(torch.int32), idx_d.to(torch.int32)
+    diff, dist = ours_nb.diff_vectors.contiguous(), ours_nb.distances.contiguous()
+    ours = AEVComputer.like_2x().to(dev)
+    g = torch.randn((1, 9999, 1008), generator=torch.Generator().manual_seed(5)).to(dev)
+
+    def ref_forward():
+        return torch.ops.cuaev.run_with_half_nbrlist(c_ref, sp32, ij32, diff, dist, comp)
+
+    def ref_fwd_bwd():
+        torch.autograd.grad(ref_forward(), c_ref, g)
+
+    def our_fwd_bwd():
+        torch.autograd.grad(ours(idx_d, c_our, cell_d, pbc_d), c_our, g)
+
+    with torch.no_grad():
+        t_aev_ref = _time_ms(ref_forward)
+        t_aev_ours = _time_ms(lambda: ours(idx_d, c_our, cell_d, pbc_d))
+    t_aev_ref_fb, t_aev_ours_fb = _time_ms(ref_fwd_bwd), _time_ms(our_fwd_bwd)
+
     # ---- networks: BmmEnsemble restated (cuBLAS) vs our tensor-core ensemble on the same AEVs
     weights = synthetic.make_weights(models.SYMBOLS_2X, synthetic.DIMS_2X, 1008, 8, seed=1234)
     model = models.from_weight_lists("2x", weights, device=dev, periodic_table_index=False)
@@ -175,6 +165,8 @@ def test_reference_gpu_path_pieces_beside_ours():
         times["tf32" if tf32 else "fp32"] = _time_ms(fwd_bwd, reps=10, warm=3)
     torch.backends.cuda.matmul.allow_tf32 = False
     rec = {"atoms": 9999, "reference_cell_list_ms": t_list_ref, "ours_cell_list_module_ms": t_list_ours,
+           "reference_cuaev_forward_ms": t_aev_ref, "reference_cuaev_forward_backward_ms": t_aev_ref_fb,
+           "ours_aev_module_forward_ms": t_aev_ours, "ours_aev_module_forward_backward_ms": t_aev_ours_fb,
            "bmm_ensemble_port_fwd_bwd_fp32_ms": times["fp32"], "bmm_ensemble_port_fwd_bwd_tf32_ms": times["tf32"],
            "note": "reference cell list = torch.ops.cell_list.cell_list built from the reference's csrc/cell_list.cpp; "
                    "network path = BmmEnsemble (nn/_infer.py:61-216) restated with torch.baddbmm (cuBLAS), forward + "

@@ -246,8 +246,9 @@ def test_bench_reference_arm_line(tmp_path):
     for k in ("impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
               "scaling", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert k in d, k
-    staged = os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "torchani")) or os.path.isdir("/root/reference/torchani")
-    # the real reference where it is staged (build container, GPU box), else the CPU port of its algorithm
+    import oracle.ref_torchani as rt
+    staged = rt.available()
+    # the real reference where it is available, else the CPU port of its algorithm
     assert d["impl"] == "reference" and d["cpu_baseline"]["kind"] == ("reference" if staged else "port")
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["cpu_baseline"]["cores"] >= 1 and d["config"]["atoms"] == 60
 
