@@ -380,6 +380,14 @@ int ani_b200_mlp_backward(const ani_mlp_model* model, float* dx, int rows_cap, c
 /*    one per window of the row tiles (all six phases of a window, then the next), sized so that a window's         */
 /*    activations stay in the L2 between the phase that writes them and the phases that read them.                  */
 int ani_b200_mlp_step_windows(const ani_mlp_model* model, int rows_cap);
+/*    Which kernel ani_b200_mlp_step launches for this model and row capacity: 0 the data-flow launch, 1 independent */
+/*    chains (ANI_B200_MLP_CHAIN=1), 2 resident chains (csrc/gemm_resident.cuh: a CTA runs one (row tile, member)     */
+/*    chain at a time with its activations and gradients in shared memory; the default where its shared-memory plan  */
+/*    fits and there are at most 8 chains per SM, ANI_B200_MLP_RESIDENT=0 / 1: never / whatever the length).          */
+int ani_b200_mlp_step_kernel(const ani_mlp_model* model, int rows_cap);
+/*    The shared-memory plan of the resident-chain kernel, bytes: out[0] resident image, out[1] weight ring of        */
+/*    layers 2-6, out[2] layer-1 ring (over both), out[3] dynamic shared memory available; out[4] 1 if it fits.       */
+int ani_b200_mlp_resident_plan(const ani_mlp_model* model, int32_t* out);
 int ani_b200_mlp_step(const ani_mlp_model* model, const void* x, float* dx, int rows_cap, const int32_t* row_atom,
                       const int32_t* layout_info, const int32_t* aev_blocks, void* act1, void* act2, void* act3,
                       float* e_member, int want_backward, int32_t* sync_i32, int32_t* status, void* stream);

@@ -92,6 +92,8 @@ _PROTOTYPES = {
     "ani_b200_half_neighbor_fill": (C.c_int, [_P, _P, _P, _P, _P, _I, _F, _P, C.c_int64, _P, _P, _P, _P, _P, _P]),
     "ani_b200_mlp_forward_backward": (C.c_int, [_P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P]),
     "ani_b200_mlp_step_windows": (C.c_int, [_P, _I]),
+    "ani_b200_mlp_step_kernel": (C.c_int, [_P, _I]),
+    "ani_b200_mlp_resident_plan": (C.c_int, [_P, _P]),
     "ani_b200_mlp_step": (C.c_int, [_P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P]),
     "ani_b200_mlp_forward": (C.c_int, [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P]),
     "ani_b200_zero_live_blocks": (C.c_int, [_P, _P, _P, _P, _P]),

@@ -85,6 +85,9 @@ __device__ __forceinline__ void tmem_ld_wait8(uint32_t (&r)[8]) {
                :
                : "memory");
 }
+__device__ __forceinline__ void sts128(uint32_t addr, const uint4& q) {
+  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(q.x), "r"(q.y), "r"(q.z), "r"(q.w) : "memory");
+}
 __device__ __forceinline__ uint32_t u4_word(const uint4& v, int i) { return i == 0 ? v.x : i == 1 ? v.y : i == 2 ? v.z : v.w; }
 
 // The epilogue of one tile, eight epilogue warps (thread = accumulator row; warps w and w + 4 share a TMEM lane quadrant
@@ -93,11 +96,16 @@ __device__ __forceinline__ uint32_t u4_word(const uint4& v, int i) { return i ==
 //   w4     shared memory, final-layer weights of this tile's columns (EPI_HEAD)
 //   y_early  the stored activation may be read before the accumulator barrier (chained launches: it is older than
 //            the launch; the data-flow launch orders it through that barrier)
+//   res      (gemm_resident.cuh) the tiled output is also written to this shared-memory image of the 128-row tile,
+//            K-block n0 / 32 + g at res + (n0 / 32 + g) * A_BLOCK_BYTES, and the four warps that complete K-block j
+//            each arrive once on res_bar[j] (after a proxy fence: the next layer's MMAs read it)
+//   c_store  false: no global stores of the tiled output (it only lives in `res`)
 template <int EPI>
 __device__ __forceinline__ void tile_epilogue_direct(const Args& args, const Tile& tl, int rt_mine, const Species& sp,
                                                      uint32_t taddr, const float* __restrict__ bias,
                                                      const float* __restrict__ w4, float* e_part, int warp, int lane,
-                                                     uint64_t* tfull_bar, uint32_t tfull_parity, float& omax, bool y_early) {
+                                                     uint64_t* tfull_bar, uint32_t tfull_parity, float& omax, bool y_early,
+                                                     unsigned char* res, uint64_t* res_bar, bool c_store) {
   static_assert(EPI == EPI_BIAS_CELU || EPI == EPI_MUL_DCELU || EPI == EPI_HEAD, "tiled-output epilogues only");
   const int quad = warp & 3, half = warp >> 2;
   const int r_tile = quad * 32 + lane;
@@ -107,6 +115,8 @@ __device__ __forceinline__ void tile_epilogue_direct(const Args& args, const Til
   const bool swapped = sw & 1u;
   const uint32_t row_base = (uint32_t)(r_tile >> 3) * 512u + (uint32_t)(r_tile & 7) * 64u;
   const bool tiled_out = EPI != EPI_HEAD || args.want_backward;
+  const bool g_out = tiled_out && c_store, s_out = tiled_out && res != nullptr;
+  const uint32_t s_row = res ? smem_u32(res) + (uint32_t)(tl.n0 / TK) * A_BLOCK_BYTES + row_base : 0u;
   const int my_row = rt_mine * TM + r_tile;
   unsigned char* ct = reinterpret_cast<unsigned char*>(args.C) +
                       ((size_t)rt_mine * args.c_kblocks + (size_t)(tl.mem * sp.c_moff + tl.n0) / TK) * A_BLOCK_BYTES + row_base;
@@ -205,8 +215,9 @@ __device__ __forceinline__ void tile_epilogue_direct(const Args& args, const Til
   auto finish = [&](int g, auto hh_c, const uint32_t (&wp)[PARTS][8]) {
     constexpr int hh = decltype(hh_c)::value;
     if (EPI == EPI_MUL_DCELU && g + 2 < ngroups) load_y(g + 2, hh, yq[hh]);
-    if (tiled_out) {
-      unsigned char* dst = ct + (size_t)g * A_BLOCK_BYTES + ((uint32_t)(hh ^ (int)(sw >> 1)) << 5);
+    const uint32_t sec = (uint32_t)(hh ^ (int)(sw >> 1)) << 5;
+    if (g_out) {
+      unsigned char* dst = ct + (size_t)g * A_BLOCK_BYTES + sec;
 #pragma unroll
       for (int p = 0; p < PARTS; ++p) {
         const uint4 lo = make_uint4(wp[p][0], wp[p][1], wp[p][2], wp[p][3]);   // columns 0-7 of the half
@@ -215,6 +226,22 @@ __device__ __forceinline__ void tile_epilogue_direct(const Args& args, const Til
           stg256(dst + p * A_PART_BYTES, hi, lo);
         else
           stg256(dst + p * A_PART_BYTES, lo, hi);
+      }
+    }
+    if (s_out) {
+      const uint32_t dst = s_row + (uint32_t)g * A_BLOCK_BYTES + sec;
+#pragma unroll
+      for (int p = 0; p < PARTS; ++p) {
+        const uint4 lo = make_uint4(wp[p][0], wp[p][1], wp[p][2], wp[p][3]);
+        const uint4 hi = make_uint4(wp[p][4], wp[p][5], wp[p][6], wp[p][7]);
+        sts128(dst + p * A_PART_BYTES, swapped ? hi : lo);
+        sts128(dst + p * A_PART_BYTES + 16, swapped ? lo : hi);
+      }
+      if (hh == 1) {
+        // K-block complete for this warp's 32 rows: generic-proxy writes -> visible to the tensor cores
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&res_bar[tl.n0 / TK + g]);
       }
     }
   };

@@ -441,7 +441,9 @@ template <int EPI>
 __device__ __forceinline__ void tile_epilogue_direct(const Args& args, const Tile& tl, int rt_mine, const Species& sp,
                                                      uint32_t taddr, const float* __restrict__ bias,
                                                      const float* __restrict__ w4, float* e_part, int warp, int lane,
-                                                     uint64_t* tfull_bar, uint32_t tfull_parity, float& omax, bool y_early);
+                                                     uint64_t* tfull_bar, uint32_t tfull_parity, float& omax, bool y_early,
+                                                     unsigned char* res = nullptr, uint64_t* res_bar = nullptr,
+                                                     bool c_store = true);
 
 // ---- the kernel -----------------------------------------------------------------------------
 template <int EPI, bool PAIR = false>

@@ -19,6 +19,7 @@
 #include "gemm_tc.cuh"
 #include "gemm_fused.cuh"
 #include "gemm_chain.cuh"
+#include "gemm_resident.cuh"
 
 namespace ani {
 
@@ -552,9 +553,70 @@ static bool use_chain_launch(const ani_mlp_model* model) {
   return ok;
 }
 
+// Shared-memory plan of the resident-chain launch (gemm_resident.cuh): the 128-row image of the widest hidden layer
+// (2 x fp16: 16 KB per 32 columns; ANI-2x 256 -> 128 KB, ANI-1x 160 -> 80 KB) plus a ring of B-only stages behind it,
+// at least two of a 256-column tile (32 KB; ANI-2x: 2, ANI-1x: 4 -- narrower layers get more, sized on the device); the
+// layer-1 forward uses a ring of A + B stages over all of it.  Two ring stages are the least that keeps the copies
+// ahead of the MMAs; 3 x bf16 operands (24 KB per K-block, 48 KB per stage) do not fit
+// that and keep the other launches.
+struct ResidentPlan {
+  bool fits;
+  int res_kb, res_bytes, small_stages, ring_bytes, big_stages;
+};
+static ResidentPlan resident_plan(const ani_mlp_model* model) {
+  ResidentPlan pl = {false, 0, 0, 0, 0, 0};
+  int hmax = 0;
+  bool widths_ok = true;
+  for (int s = 0; s < model->num_species; ++s) {
+    const ani_mlp_species& p = model->sp[s];
+    hmax = max(hmax, max(p.h1, max(p.h2, p.h3)));
+    widths_ok = widths_ok && p.h1 <= tc::TN_MAX && p.h2 <= tc::TN_MAX && p.h3 <= tc::TN_MAX;
+  }
+  pl.res_kb = (hmax + tc::TK - 1) / tc::TK;
+  pl.res_bytes = pl.res_kb * tc::A_BLOCK_BYTES;
+  pl.small_stages = min(tc::MAX_STAGES, max(0, tc::RES_AVAIL - pl.res_bytes) / tc::RES_B_STAGE_BYTES);
+  pl.ring_bytes = pl.small_stages * tc::RES_B_STAGE_BYTES;
+  pl.big_stages = min(tc::MAX_STAGES, tc::RES_AVAIL / tc::CHAIN_STAGE_BYTES);
+  pl.fits = widths_ok && hmax > 0 && pl.small_stages >= 2 && pl.big_stages >= 2;
+  return pl;
+}
+
+// Where the plan fits (the opt-in ANI_B200_MLP_CHAIN=1 comes first), for lists of at most 8 chains per SM;
+// ANI_B200_MLP_RESIDENT=0 / 1: never / whatever the length.  Measured on B200 (1000 W, profiles/r03_bench_*), MLP
+// stage against the data-flow launch / chained launches: water 999 atoms (0.5 chains per SM) 58 vs 82 us, gdb256 121
+// vs 144 us, water 9 999 atoms (4.3 per SM) 185 vs 202 us; protein in water 50 k atoms (21 per SM) 1.20 vs 1.12 ms.
+static bool use_resident_launch(const ani_mlp_model* model, int rows_cap) {
+  if (use_chain_launch(model) || !resident_plan(model).fits) return false;
+  const char* e = getenv("ANI_B200_MLP_RESIDENT");
+  if (e) return atoi(e) != 0;
+  static int num_sms = 0;
+  if (num_sms == 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+      num_sms = 148;   // (host-only callers: a B200)
+  }
+  return (long long)(rows_cap / ANI_TILE_ROWS) * model->num_members <= 8LL * num_sms;
+}
+
+extern "C" int ani_b200_mlp_resident_plan(const ani_mlp_model* model, int32_t* out) {
+  if (!model || !out || model->num_species < 1 || model->num_species > ANI_MAX_SPECIES) return ANI_ERR_BAD_ARG;
+  const ResidentPlan pl = resident_plan(model);
+  out[0] = pl.res_bytes;
+  out[1] = pl.ring_bytes;
+  out[2] = pl.big_stages * tc::CHAIN_STAGE_BYTES;
+  out[3] = tc::RES_AVAIL;
+  out[4] = pl.fits ? 1 : 0;
+  return ANI_OK;
+}
+
+extern "C" int ani_b200_mlp_step_kernel(const ani_mlp_model* model, int rows_cap) {
+  if (!model) return ANI_ERR_BAD_ARG;
+  return use_chain_launch(model) ? 1 : use_resident_launch(model, rows_cap) ? 2 : 0;
+}
+
 extern "C" int ani_b200_mlp_step_windows(const ani_mlp_model* model, int rows_cap) {
   if (!model || rows_cap < ANI_TILE_ROWS) return 1;
-  if (use_chain_launch(model)) return 1;   // independent chains: one launch whatever the size
+  if (use_chain_launch(model) || use_resident_launch(model, rows_cap)) return 1;   // independent chains: one launch
   // Experiment (measured on B200, 9 999 atoms: 214 / 305 / 387 / 479 us for 1 / 2 / 3 / 4 windows): every launch of the
   // phase-major kernel costs ~90 us of dependency ramp before its ~4.9 us per unit and CTA, far more than the L2
   // residency of a window buys -- one window unless the environment asks for more
@@ -591,6 +653,30 @@ extern "C" int ani_b200_mlp_step(const ani_mlp_model* model, const void* x, floa
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&num_sms_c, cudaDevAttrMultiProcessorCount, dev);
     cudaFuncSetAttribute(tc::k_mlp_chain<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::FUSED_SMEM_BYTES);
+  }
+  // resident chains (gemm_resident.cuh): one launch, a chain's activations and gradients in shared memory
+  if (use_resident_launch(model, rows_cap)) {
+    static tc::ResidentArgs RA;
+    static bool attr_set = false;
+    if (!attr_set) {
+      cudaFuncSetAttribute(tc::k_mlp_resident, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::FUSED_SMEM_BYTES);
+      attr_set = true;
+    }
+    const ResidentPlan pl = resident_plan(model);
+    RA.n_phases = want_backward ? 6 : 3;
+    RA.res_kb = pl.res_kb;
+    static const int epis_r[6] = {tc::EPI_BIAS_CELU, tc::EPI_BIAS_CELU, tc::EPI_HEAD, tc::EPI_MUL_DCELU, tc::EPI_MUL_DCELU,
+                                  tc::EPI_PLAIN};
+    for (int p = 0; p < tc::MAX_PHASES; ++p) {
+      RA.epi[p] = epis_r[p];
+      RA.ph[p] = base;
+      fill_phase(RA.ph[p], p, model, x, dx, act1, act2, act3, e_member, aev_blocks, want_backward, rows_cap, 1);
+      RA.ph[p].allow_narrow = 0;   // one column tile per member in phases 0-4 (the layer-1 backward: any number)
+    }
+    if (want_backward) launch_zero_compact(model, (want_backward == 1 && M > 1) ? dx : nullptr, layout_info, aev_blocks, st);
+    tc::k_mlp_resident<<<num_sms_c, tc::CHAIN_THREADS, tc::FUSED_SMEM_BYTES, st>>>(RA);
+    ANI_CUDA_CHECK_LAUNCH();
+    return ANI_OK;
   }
   // independent chains (gemm_chain.cuh): one launch, no synchronisation between CTAs.  ANI_B200_MLP_CHAIN=0: the
   // phase-major data-flow launch below; ANI_B200_CHAIN_DEPTH: chains a CTA interleaves

@@ -501,6 +501,11 @@ class Engine:
         # 0.235 ms); for short lists (< 3 waves) the chained launches win, a launch boundary being a cheaper hand-over
         # of a row tile than an L2 counter when the six-layer chain is exposed.  "auto" applies exactly that rule;
         # ANI_B200_MLP_FUSED=0 / 1 forces one of them.
+        # A third schedule runs inside ani_b200_mlp_step wherever it fits (mlp_schedule): resident chains
+        # (csrc/gemm_resident.cuh), each (row tile, member) chain on one SM with its activations and gradients in
+        # shared memory, up to 8 chains per SM.  Measured on B200 (1000 W, profiles/r03_bench_*), step against the
+        # previous choice: water 999 atoms 0.115 vs 0.138 ms, gdb256 0.230 vs 0.252 ms, water 9 999 atoms 0.323 vs
+        # 0.346 ms; the protein-in-water box of 50 k atoms (21 chains per SM) keeps the data-flow launch.
         self.mlp_mode = os.environ.get("ANI_B200_MLP_FUSED", "auto")
         self._num_sms = torch.cuda.get_device_properties(self.device).multi_processor_count
         self._side_stream: tp.Optional[torch.cuda.Stream] = None
@@ -606,7 +611,7 @@ class Engine:
         # prepare 1 (+1 grid kernel for open single systems), AEV fwd 1, GEMM fwd 3,
         # (zero + GEMM bwd 3 + AEV bwd 1), reduce 1
         mlp = ((self.lib.ani_b200_mlp_step_windows(C.byref(self.nets.model), ws.rows_cap) + (1 if want_grad else 0))
-               if self._use_dataflow_mlp(hi - lo) else (3 + (4 if want_grad else 0)))
+               if self._use_dataflow_mlp(hi - lo, ws.rows_cap) else (3 + (4 if want_grad else 0)))
         self.launches_per_step = 1 + (0 if (pbc or n_conf > 1) else 1) + 1 + mlp + (1 if want_grad else 0) + 1
         grad = ws.grad.view(n_conf, n_per_conf, 3) if want_grad else None
         virial = ws.virial.sum(0).view(3, 3) if want_virial else None
@@ -672,7 +677,7 @@ class Engine:
                 ptr(ws.species_i32), n, lo, hi, n_conf, n_per_conf, ptr(self.sae), ptr(ws.atomic),
                 ptr(ws.member_atomic), ws.energies_ptr, stream_handle)
 
-        self.mlp_fused = self._use_dataflow_mlp(hi - lo)
+        self.mlp_fused = self._use_dataflow_mlp(hi - lo, ws.rows_cap)
         if not split and self.mlp_fused:
             # the six GEMMs of the step as ONE persistent data-flow launch (csrc/gemm_fused.cuh)
             self._timed("mlp_forward_backward", lambda: L.ani_b200_mlp_step(
@@ -788,13 +793,23 @@ class Engine:
             e_m = e_m + self.sae[sp].masked_fill(species < 0, 0.0).sum(-1).unsqueeze(0)
         return e_m, grads.view(len(active), n_conf, n_per_conf, 3)
 
-    def _use_dataflow_mlp(self, owned: int) -> bool:
-        """One data-flow launch (True) or six chained launches (False) for `owned` atoms; see __init__."""
-        if self.mlp_mode in ("0", "1"):
-            return self.mlp_mode == "1"
+    def mlp_schedule(self, owned: int, rows_cap: int) -> str:
+        """How the MLP of a step over `owned` atoms (workspace of `rows_cap` rows) runs: "resident" (one launch of
+        csrc/gemm_resident.cuh), "dataflow" (one launch of csrc/gemm_fused.cuh; "chains" with ANI_B200_MLP_CHAIN=1) or
+        "chained" (six launches); see __init__.  ani_b200_mlp_step picks its kernel itself (ani_b200_mlp_step_kernel)."""
+        if self.mlp_mode == "0":
+            return "chained"
+        kernel = self.lib.ani_b200_mlp_step_kernel(C.byref(self.nets.model), rows_cap)
+        step = {0: "dataflow", 1: "chains", 2: "resident"}[kernel]
+        if self.mlp_mode == "1" or step == "resident":
+            return step
         units = (-(-owned // TILE) + 1) * self.nets.num_members     # per layer: row tiles x members (>= 1 column tile)
         waves = units / self._num_sms
-        return waves >= 3.0 and waves / math.ceil(waves) < 0.9
+        return step if waves >= 3.0 and waves / math.ceil(waves) < 0.9 else "chained"
+
+    def _use_dataflow_mlp(self, owned: int, rows_cap: int) -> bool:
+        """One launch of ani_b200_mlp_step (True) or six chained launches (False) for `owned` atoms."""
+        return self.mlp_schedule(owned, rows_cap) != "chained"
 
     def note_composition(self, ws: Workspace) -> None:
         """Before a graph capture (the shape has already run eagerly): read the element mask of the last
